@@ -9,6 +9,7 @@
     python bench.py --mode fwd_loss      # BASELINE configs[2]: forward + full-softmax loss only
     python bench.py --mode sampled       # BASELINE configs[3]: train step with sampled softmax (25 negatives)
     python bench.py --workload large     # BASELINE configs[4]'s model: 3M/2M vocab, d=256 (run it with --gpus 8)
+    python bench.py --dump-outputs DIR   # also write what the last timed step computed to DIR/*.npy (see dump_outputs)
 
 A "step" is one pass of the hot path over one batch of synthetic path-context bags: three
 embedding gathers, tanh(x.W), masked softmax attention, full-softmax logits + loss, the whole
@@ -51,6 +52,7 @@ NUM_SAMPLED = 25      # BASELINE.json configs[2]: "sampled_softmax (neg=25)"
 NVLINK_PEER_GBS = 770.0   # measured peer copy per direction per GPU (/opt/skills/guides/B200_PROFILING.md)
 N_BATCHES = 16        # distinct input batches the timed loop cycles through
 REFERENCE_BUDGET_S = 240.0   # --impl reference: most CPU seconds the timed + warm-up steps may take
+DUMP_TABLE_BYTES = 16 << 20  # --dump-outputs: most bytes written per embedding table (a seeded sample of its rows)
 
 
 def workload_string(name, w, mode):
@@ -207,6 +209,31 @@ def sampled_inputs(w, batch, seed):
     return sampled, logq(batch[4]), logq(sampled)
 
 
+def dump_outputs(out_dir, eng, mode, loss, code=None):
+    """Writes what a caller of the timed step holds after its last step, as float32 DIR/<name>.npy: `loss` ([1]); for
+    the train modes the parameters that step left behind (W and a whole; of tok, path and tgt the rows drawn by
+    np.random.default_rng(0) without replacement, sorted, at most DUMP_TABLE_BYTES per table); for fwd_loss the code
+    vectors `code` [B, D].  The inputs and the initialisation are seeded, so two builds run with the same arguments can
+    be compared array for array."""
+    import torch
+    out = {"loss": loss}
+    if mode == "fwd_loss":
+        out["code"] = code
+    else:
+        eng.sync_tables()                # lazy Adam: bring every deferred row up to date before it is read
+        for k in ("tok", "path", "tgt", "W", "a"):
+            p = eng.params[k]
+            if k in ("W", "a"):
+                out[k] = p
+                continue
+            n, row_bytes = p.shape[0], p.shape[1] * 4
+            rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_TABLE_BYTES // row_bytes), replace=False))
+            out[k] = p.index_select(0, torch.from_numpy(rows).to(p.device))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ================================ our arm ========================================================
 def run_ours(args):
     import torch
@@ -227,6 +254,8 @@ def run_ours(args):
     mode = args.mode
     if world > 1 and mode != "train":
         raise SystemExit("--mode %s is a single-GPU workload (BASELINE configs[1]/[2])" % mode)
+    if world > 1 and args.dump_outputs:
+        raise SystemExit("--dump-outputs is single-GPU (the multi-GPU schedules keep the tables in row shards)")
 
     w = dict(WORKLOADS[args.workload])
     if args.batch:
@@ -275,6 +304,7 @@ def run_ours(args):
     pinned = [[torch.from_numpy(np.ascontiguousarray(a)).pin_memory() for a in b] for b in host]
     devb = [[t.to(dev) for t in b] for b in pinned]
     stage = [torch.empty_like(t, device=dev) for t in pinned[0]]      # e2e: this step's inputs are copied here
+    last_code = [None]                                                  # fwd_loss: the code vectors of the latest step
 
     def step_dev(i):
         b = devb[i % n_batches]
@@ -283,6 +313,7 @@ def run_ours(args):
         if mode == "sampled":
             return trainer.step_device_sampled(*b)
         code, _ = eng.forward(b[0], b[1], b[2], b[3], want_attention=False)
+        last_code[0] = code
         return eng.loss(code, b[4])
 
     loss_pin = torch.zeros(1, dtype=torch.float32).pin_memory()
@@ -358,6 +389,9 @@ def run_ours(args):
     eng.set_option("profile", 0)
     clk = clocks.stop(t_wall0, t_wall1) if rank == 0 else None
     last_loss = float(loss_dev.cpu()[0])
+    if args.dump_outputs:
+        # before the e2e and 3xTF32 passes below train the model further
+        dump_outputs(args.dump_outputs, eng, mode, loss_dev, last_code[0])
 
     # ---- end to end through the host-buffer API (e2e) ---------------------------------------
     ms_e2e, _ = timed(step_e2e, K, 2)
@@ -690,7 +724,12 @@ def main():
                     help="tcgen05 GEMMs as CTA pairs (cta_group::2): 0 never, 1 always, 2 auto (default)")
     ap.add_argument("--dp-schedule", default=os.environ.get("C2V_DP_SCHEDULE", "fully_sharded"),
                     choices=["fully_sharded", "table_sharded", "sharded", "allreduce"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32, < 64 MB; "
+                         "single GPU, our arm)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the CUDA engine computed (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
