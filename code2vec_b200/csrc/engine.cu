@@ -1461,6 +1461,7 @@ int c2v_get_option(const c2v_engine* e, const char* key, int64_t* value) {
   if (!strcmp(key, "lazy_adam")) { *value = e->lazy; return C2V_OK; }
   if (!strcmp(key, "adam_sweep_period")) { *value = e->sweep_period; return C2V_OK; }
   if (!strcmp(key, "adam_rest_shortcut")) { *value = e->rest_shortcut; return C2V_OK; }
+  if (!strcmp(key, "adam_rows_occupancy")) { *value = e->adam_rows_occ; return C2V_OK; }
   if (!strcmp(key, "cta_pair")) { *value = e->cta_pair; return C2V_OK; }
   if (!strcmp(key, "dy_late")) { *value = e->dy_late; return C2V_OK; }
   if (!strcmp(key, "fuse_target_adam")) { *value = e->fuse_tgt; return C2V_OK; }
