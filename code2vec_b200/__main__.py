@@ -8,6 +8,11 @@ extractor's output format, SURVEY A.5) from `--predict_input FILE` or standard i
 them as extractor.py:22-38 does (first MAX_CONTEXTS contexts, path strings replaced by their Java
 `String.hashCode`, padding to MAX_CONTEXTS fields) and prints each prediction in the reference's layout
 (interactive_predict.py:50-63), attention paths un-hashed when the input carried path strings.
+
+`--most_similar target|token [--similar_input FILE] [--topn N]` answers gensim `most_similar` queries (the workflow
+the reference README runs on the --save_t2v / --save_w2v files, README.md:236-251) on the GPU: one query per line
+of FILE or standard input, positive words separated by spaces, then optionally a TAB and the negative words.  The
+extra flags are taken out of the argument list before `Config` parses it, so config.py stays the reference's.
 """
 from __future__ import annotations
 
@@ -74,13 +79,75 @@ def print_predictions(config: Config, model, lines: Iterable[str], out=None):
             out.write(" ".join(map(str, raw.code_vector)) + "\n")
 
 
+SIMILARITY_VOCABS = {"target": VocabType.Target, "token": VocabType.Token}
+
+
+def parse_similarity_line(line: str):
+    """One nearest-neighbour query line -> (positive words, negative words), or None for a blank line.  Positive
+    words are separated by spaces; an optional TAB is followed by the negative words.  (A `-` prefix cannot mark a
+    negative word: nothing in the extractor's token normalisation rules out a token that starts with `-`.)"""
+    line = line.rstrip("\r\n")
+    pos, _, neg = line.partition("\t")
+    positive, negative = pos.split(), neg.split()
+    if not positive and not negative:
+        return None
+    return positive, negative
+
+
+def print_similar(model, lines: Iterable[str], vocab_type: VocabType, topn: int, out=None):
+    """gensim's most_similar for every query line (reference README.md:236-251), printed in print_predictions'
+    layout: `Query:` then one `\\t(score) word` line per hit.  A line with an unknown word prints one error line."""
+    from .b200_model import similarity_query_terms
+    out = sys.stdout if out is None else out
+    vocab = model.vocabs.get(vocab_type)
+    entries = []                                       # (line, query or None, error message or None)
+    for line in lines:
+        q = parse_similarity_line(line)
+        if q is None:
+            continue
+        try:
+            similarity_query_terms(vocab, *q)
+            entries.append((line.rstrip("\r\n"), q, None))
+        except (KeyError, ValueError) as exc:
+            entries.append((line.rstrip("\r\n"), None, exc.args[0] if exc.args else str(exc)))
+    valid = [q for _, q, _ in entries if q is not None]
+    results = iter(model.most_similar_many(valid, topn=topn, vocab_type=vocab_type) if valid else [])
+    for line, q, err in entries:
+        out.write("Query:\t" + line + "\n")
+        if err is not None:
+            out.write("Error:\t%s\n" % err)
+            continue
+        for word, score in next(results):
+            out.write("\t(%f) %s\n" % (score, word))
+
+
+def _pop_flag(argv, flag: str):
+    """Removes `flag VALUE` from argv and returns VALUE (None when absent)."""
+    if flag not in argv:
+        return None
+    i = argv.index(flag)
+    if i + 1 >= len(argv):
+        raise SystemExit("%s needs a value" % flag)
+    value = argv[i + 1]
+    del argv[i:i + 2]
+    return value
+
+
+def strip_extra_flags(argv):
+    """Takes the flags the reference does not have out of argv before Config parses the rest:
+    {"predict_input": FILE, "most_similar": "target" | "token", "similar_input": FILE, "topn": int}."""
+    argv = list(argv)
+    extra = {"predict_input": _pop_flag(argv, "--predict_input"), "most_similar": _pop_flag(argv, "--most_similar"),
+             "similar_input": _pop_flag(argv, "--similar_input"), "topn": _pop_flag(argv, "--topn")}
+    if extra["most_similar"] is not None and extra["most_similar"] not in SIMILARITY_VOCABS:
+        raise SystemExit("--most_similar must be one of: %s" % ", ".join(sorted(SIMILARITY_VOCABS)))
+    extra["topn"] = 10 if extra["topn"] is None else int(extra["topn"])
+    return argv, extra
+
+
 def main(argv: Optional[Iterable[str]] = None) -> int:
-    argv = list(sys.argv[1:] if argv is None else argv)
-    predict_input = None
-    if "--predict_input" in argv:                      # the one flag the reference does not have
-        i = argv.index("--predict_input")
-        predict_input = argv[i + 1]
-        del argv[i:i + 2]
+    argv, extra = strip_extra_flags(sys.argv[1:] if argv is None else argv)
+    predict_input = extra["predict_input"]
     config = Config(set_defaults=True)
     config.load_from_args(argv)
     config.verify()
@@ -106,6 +173,13 @@ def main(argv: Optional[Iterable[str]] = None) -> int:
                     print_predictions(config, model, f)
             else:
                 print_predictions(config, model, sys.stdin)
+        if extra["most_similar"] is not None:
+            vocab_type = SIMILARITY_VOCABS[extra["most_similar"]]
+            if extra["similar_input"]:
+                with open(extra["similar_input"], "r") as f:
+                    print_similar(model, f, vocab_type, extra["topn"])
+            else:
+                print_similar(model, sys.stdin, vocab_type, extra["topn"])
     finally:
         model.close_session()
     return 0

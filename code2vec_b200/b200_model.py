@@ -16,7 +16,7 @@ import struct
 import time
 from collections import Counter
 from functools import partial
-from typing import Dict, Iterable, List, Optional
+from typing import Dict, Iterable, List, Optional, Tuple
 
 import numpy as np
 
@@ -80,6 +80,35 @@ def _with_next(iterable):
         yield cur, nxt
         cur = nxt
     yield cur, None
+
+
+def similarity_query_terms(vocab, positive=None, negative=None):
+    """A most_similar query -> ([(row or vector, +1 / -1)], [rows of the query's words]).  As gensim: a single word
+    or vector may stand for a one-item list, vectors are not excluded from the results, a word outside the
+    vocabulary raises KeyError (it is not mapped to the OOV word) and a query without items raises ValueError."""
+    def as_list(items):
+        if items is None:
+            return []
+        if isinstance(items, (str, np.ndarray)):
+            return [items]
+        return list(items)
+    terms, exclude = [], []
+    for items, weight in ((as_list(positive), 1.0), (as_list(negative), -1.0)):
+        for item in items:
+            if isinstance(item, str):
+                if item not in vocab.word_to_index:
+                    raise KeyError("word '%s' not in vocabulary" % item)
+                row = int(vocab.word_to_index[item])
+                terms.append((row, weight))
+                if row not in exclude:
+                    exclude.append(row)
+            else:
+                terms.append((np.asarray(item, dtype=np.float32).reshape(-1), weight))
+    if not terms:
+        raise ValueError("cannot compute similarity with no input")
+    if len(terms) > PathAttentionEngine.MAX_QUERY_TERMS:
+        raise ValueError("at most %d words / vectors per query" % PathAttentionEngine.MAX_QUERY_TERMS)
+    return terms, exclude
 
 
 _CKPT_MAGIC = b"C2VB200\0"
@@ -366,6 +395,50 @@ class Code2VecModel(Code2VecModelBase):
                 topk_predicted_words_scores=scores[0], attention_per_context=attention_per_context,
                 code_vector=(code_vectors[0] if self.config.EXPORT_CODE_VECTORS else None)))
         return results
+
+    # ---- nearest neighbours: gensim's KeyedVectors.most_similar on the resident tables ----------------------
+    # The reference README (README.md:236-251) loads the --save_t2v / --save_w2v text files into gensim for these
+    # queries; here the cosine scan and top-k run on the engine (c2v_compose_queries, c2v_nearest).
+    def most_similar(self, positive=None, negative=None, topn: int = 10, vocab_type: VocabType = VocabType.Target,
+                     restrict_vocab: Optional[int] = None) -> List[Tuple[str, float]]:
+        """gensim's most_similar: the `topn` rows closest by cosine to unitvec(mean of the unit vectors of the positive
+        words and the negated unit vectors of the negative ones).  Items may be words or numpy vectors (used as given,
+        not excluded); the query's words are never returned.  restrict_vocab=N scans the first N rows only (the N most
+        frequent words).  Unknown words raise KeyError, an empty query ValueError."""
+        return self.most_similar_many([(positive, negative)], topn=topn, vocab_type=vocab_type,
+                                      restrict_vocab=restrict_vocab)[0]
+
+    def similar_by_vector(self, vector, topn: int = 10, vocab_type: VocabType = VocabType.Target,
+                          restrict_vocab: Optional[int] = None) -> List[Tuple[str, float]]:
+        """The names (or tokens) closest to a vector, e.g. a code vector from predict()."""
+        return self.most_similar(positive=[np.asarray(vector, dtype=np.float32)], topn=topn, vocab_type=vocab_type,
+                                 restrict_vocab=restrict_vocab)
+
+    def most_similar_many(self, queries, topn: int = 10, vocab_type: VocabType = VocabType.Target,
+                          restrict_vocab: Optional[int] = None) -> List[List[Tuple[str, float]]]:
+        """most_similar for many (positive, negative) queries: one query-composition launch and one search launch
+        serve them all."""
+        vocab = self.vocabs.get(vocab_type)
+        parsed = [similarity_query_terms(vocab, pos, neg) for pos, neg in queries]
+        if not parsed:
+            return []
+        if not 1 <= int(topn) <= PathAttentionEngine.NEAREST_MAX_K:
+            raise ValueError("topn must be in [1, %d]" % PathAttentionEngine.NEAREST_MAX_K)
+        e = self.engine
+        name = self._param_of_vocab[vocab_type]
+        if getattr(e, "table_world", 1) > 1 and name != "tgt":
+            raise NotImplementedError("most_similar over row-sharded token / path tables is not supported")
+        e.sync_tables()                          # lazy Adam: deferred rows must be current before they are scanned
+        table = e.params[name]
+        queries_dev = e.compose_queries(table, [terms for terms, _ in parsed])   # query words may lie past restrict_vocab
+        bank = table if restrict_vocab is None else table[:max(1, min(int(restrict_vocab), table.shape[0]))]
+        n_ex = max([len(ex) for _, ex in parsed] + [1])
+        exclude = np.full((len(parsed), n_ex), -1, dtype=np.int32)
+        for q, (_, ex) in enumerate(parsed):
+            exclude[q, :len(ex)] = ex
+        idx, val = e.nearest(bank, queries_dev, int(topn), exclude=exclude)
+        idx, val = idx.cpu().numpy(), val.cpu().numpy()
+        return [[(vocab.index_to_word[int(i)], float(v)) for i, v in zip(ri, rv) if i >= 0] for ri, rv in zip(idx, val)]
 
     def _get_vocab_embedding_as_np_array(self, vocab_type: VocabType) -> np.ndarray:
         assert vocab_type in VocabType

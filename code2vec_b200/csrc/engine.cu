@@ -18,6 +18,7 @@
 #include "umma_gemm.cuh"
 #include "umma_gemm2.cuh"
 #include "ctx_fused.cuh"
+#include "similarity.cuh"
 
 using namespace c2v;
 
@@ -1224,6 +1225,44 @@ int adam_impl(c2v_engine* e, cudaStream_t st, float lr, float b1, float b2, floa
   return C2V_OK;
 }
 
+// ---- nearest-neighbour search (similarity.cuh) ----------------------------------------------------
+// Touches neither the workspace nor any engine state: a search between two train steps leaves the next step unchanged.
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+int check_bank(c2v_engine* e, const float* bank, int64_t rows, int32_t dim) {
+  if (!bank) return fail(e, C2V_ERR_INVALID, "bank is NULL");
+  if (rows < 1 || rows > INT32_MAX) return fail(e, C2V_ERR_INVALID, "rows must be in [1, 2^31)");
+  if (dim < 4 || dim > 1024 || dim % 4) return fail(e, C2V_ERR_INVALID, "dim must be a multiple of 4 in [4, 1024]");
+  if (!aligned16(bank)) return fail(e, C2V_ERR_INVALID, "bank must be 16-byte aligned");
+  return C2V_OK;
+}
+
+template <int QB>
+int launch_nearest(c2v_engine* e, cudaStream_t st, const float* bank, int rows, int dim, const float* queries, int n, int k,
+                   const int32_t* exclude, int n_exclude, const sim::Layout& L, int slices, ValIdx* cand) {
+  C2V_CUDA(e, cudaFuncSetAttribute(sim::nearest_kernel<QB>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
+  const dim3 grid((unsigned)((n + L.qc - 1) / L.qc), (unsigned)slices);
+  C2V_LAUNCH(e, (sim::nearest_kernel<QB><<<grid, sim::kThreads, L.total, st>>>(bank, rows, dim, queries, n, k, exclude,
+                                                                                n_exclude, L, cand)));
+  return C2V_OK;
+}
+
+int nearest_impl(c2v_engine* e, cudaStream_t st, const float* bank, int rows, int dim, const float* queries, int n, int k,
+                 const int32_t* exclude, int n_exclude, int32_t* idx, float* val, void* scratch) {
+  const sim::Layout L = sim::make_layout(dim, k);
+  const int slices = sim::slices_for(rows);
+  ValIdx* cand = reinterpret_cast<ValIdx*>(scratch);
+  // register block of 1, 2, 4 or 8 queries: a single query does not pay for seven zero ones
+  int rc;
+  if (n == 1) rc = launch_nearest<1>(e, st, bank, rows, dim, queries, n, k, exclude, n_exclude, L, slices, cand);
+  else if (n == 2) rc = launch_nearest<2>(e, st, bank, rows, dim, queries, n, k, exclude, n_exclude, L, slices, cand);
+  else if (n <= 4) rc = launch_nearest<4>(e, st, bank, rows, dim, queries, n, k, exclude, n_exclude, L, slices, cand);
+  else rc = launch_nearest<8>(e, st, bank, rows, dim, queries, n, k, exclude, n_exclude, L, slices, cand);
+  if (rc) return rc;
+  C2V_LAUNCH(e, (sim::merge_kernel<<<n, kTopkThreads, 0, st>>>(cand, slices, k, idx, val)));
+  return C2V_OK;
+}
+
 }  // namespace
 
 // ================================== C ABI =======================================================
@@ -1505,6 +1544,49 @@ int c2v_topk(c2v_engine* e, const float* code_vec, int32_t B, int32_t* idx, floa
   if (!code_vec || !idx || !val) return fail(e, C2V_ERR_INVALID, "NULL argument");
   C2V_CUDA(e, cudaSetDevice(e->device));
   return topk_impl(e, (cudaStream_t)stream, code_vec, B, idx, val, normalize);
+}
+
+size_t c2v_nearest_scratch_bytes(int64_t rows, int32_t n, int32_t k) {
+  if (rows < 1 || rows > INT32_MAX || n < 1 || k < 1 || k > sim::kMaxK) return 0;
+  return (size_t)n * (size_t)sim::slices_for(rows) * (size_t)k * sizeof(ValIdx);
+}
+
+int c2v_compose_queries(c2v_engine* e, const float* bank, int64_t rows, int32_t dim, const int32_t* term_rows,
+                        const float* term_weights, const float* term_vectors, int32_t n, int32_t max_terms,
+                        float* queries, void* stream) {
+  if (!e) return C2V_ERR_INVALID;
+  int rc = check_bank(e, bank, rows, dim);
+  if (rc) return rc;
+  if (!term_rows || !term_weights || !queries) return fail(e, C2V_ERR_INVALID, "NULL argument");
+  if (n < 1) return fail(e, C2V_ERR_INVALID, "n must be >= 1");
+  if (max_terms < 1 || max_terms > sim::kMaxTerms) return fail(e, C2V_ERR_INVALID, "max_terms must be in [1, 16]");
+  if (!aligned16(queries) || (term_vectors && !aligned16(term_vectors)))
+    return fail(e, C2V_ERR_INVALID, "queries / term_vectors must be 16-byte aligned");
+  C2V_CUDA(e, cudaSetDevice(e->device));
+  C2V_LAUNCH(e, (sim::compose_kernel<<<n, sim::kThreads, 0, (cudaStream_t)stream>>>(bank, rows, dim, term_rows, term_weights,
+                                                                                     term_vectors, max_terms, queries)));
+  return C2V_OK;
+}
+
+int c2v_nearest(c2v_engine* e, const float* bank, int64_t rows, int32_t dim, const float* queries, int32_t n, int32_t k,
+                const int32_t* exclude, int32_t n_exclude, int32_t* idx, float* val, void* scratch, size_t scratch_bytes,
+                void* stream) {
+  if (!e) return C2V_ERR_INVALID;
+  int rc = check_bank(e, bank, rows, dim);
+  if (rc) return rc;
+  if (!queries || !idx || !val || !scratch) return fail(e, C2V_ERR_INVALID, "NULL argument");
+  if (n < 1) return fail(e, C2V_ERR_INVALID, "n must be >= 1");
+  if (k < 1 || k > sim::kMaxK) return fail(e, C2V_ERR_INVALID, "k must be in [1, 64]");
+  if (n_exclude < 0 || n_exclude > sim::kMaxExclude) return fail(e, C2V_ERR_INVALID, "n_exclude must be in [0, 16]");
+  if (n_exclude > 0 && !exclude) return fail(e, C2V_ERR_INVALID, "exclude is NULL with n_exclude > 0");
+  if (!aligned16(queries)) return fail(e, C2V_ERR_INVALID, "queries must be 16-byte aligned");
+  if (!aligned16(scratch)) return fail(e, C2V_ERR_INVALID, "scratch must be 16-byte aligned");
+  if (reinterpret_cast<uintptr_t>(idx) % 4 || reinterpret_cast<uintptr_t>(val) % 4)
+    return fail(e, C2V_ERR_INVALID, "idx / val must be 4-byte aligned");
+  if (scratch_bytes < c2v_nearest_scratch_bytes(rows, n, k))
+    return fail(e, C2V_ERR_INVALID, "scratch smaller than c2v_nearest_scratch_bytes()");
+  C2V_CUDA(e, cudaSetDevice(e->device));
+  return nearest_impl(e, (cudaStream_t)stream, bank, (int)rows, dim, queries, n, k, exclude, n_exclude, idx, val, scratch);
 }
 
 int c2v_loss(c2v_engine* e, const float* code_vec, const int32_t* target, int32_t B, float* loss_out, void* stream) {

@@ -62,6 +62,9 @@ _SIGNATURES = {
     "c2v_forward": (C.c_int, [_P, _P, _P, _P, _P, _I32, _P, _P, _P]),
     "c2v_topk": (C.c_int, [_P, _P, _I32, _P, _P, _I32, _P]),
     "c2v_loss": (C.c_int, [_P, _P, _P, _I32, _P, _P]),
+    "c2v_nearest_scratch_bytes": (C.c_size_t, [C.c_int64, _I32, _I32]),
+    "c2v_compose_queries": (C.c_int, [_P, _P, C.c_int64, _I32, _P, _P, _P, _I32, _I32, _P, _P]),
+    "c2v_nearest": (C.c_int, [_P, _P, C.c_int64, _I32, _P, _I32, _I32, _P, _I32, _P, _P, _P, C.c_size_t, _P]),
     "c2v_train_step": (C.c_int, [_P, _P, _P, _P, _P, _P, _I32, C.c_float, C.c_uint64, C.c_uint64, _P, _P, _P]),
     "c2v_sampled_train_step": (C.c_int, [_P, _P, _P, _P, _P, _P, _I32, _P, _I32, _P, _P, C.c_float,
                                          C.c_uint64, C.c_uint64, _P, _P, _P]),
@@ -394,6 +397,78 @@ class PathAttentionEngine:
         val = torch.empty((B, k), dtype=torch.float32, device=self.dev)
         self._check(self.lib.c2v_topk(self.h, code_vec.data_ptr(), B, idx.data_ptr(), val.data_ptr(),
                                       int(normalize), self._stream()))
+        return idx, val
+
+    # ---- nearest-neighbour search (c2v_compose_queries / c2v_nearest) ---------------------------------
+    NEAREST_MAX_K = 64
+    NEAREST_MAX_EXCLUDE = 16
+    MAX_QUERY_TERMS = 16
+
+    @staticmethod
+    def nearest_query_capacity(dim: int) -> int:
+        """Queries c2v_nearest keeps in shared memory per chunk at this width (similarity.cuh, query_capacity): the
+        bank is read once per chunk."""
+        return min(64, max(8, (32768 // (int(dim) * 4)) // 8 * 8))
+
+    def compose_queries(self, bank, terms):
+        """gensim's query vectors for word queries: terms = one list per query of (row or vector, weight) pairs, a row
+        being an int index into `bank` (unit-normalised before weighting) and a vector a 1-D array / tensor of
+        bank.shape[1] floats used as given.  Returns a device tensor [n, dim] of unit vectors (c2v_compose_queries)."""
+        torch = self.torch
+        n, dim = len(terms), int(bank.shape[1])
+        mt = max([len(t) for t in terms] + [1])
+        if mt > self.MAX_QUERY_TERMS:
+            raise ValueError("at most %d terms per query" % self.MAX_QUERY_TERMS)
+        rows = np.full((n, mt), -1, dtype=np.int32)
+        weights = np.zeros((n, mt), dtype=np.float32)
+        vecs = None
+        for q, query in enumerate(terms):
+            for t, (term, w) in enumerate(query):
+                weights[q, t] = float(w)
+                if isinstance(term, (int, np.integer)):
+                    if not 0 <= int(term) < bank.shape[0]:
+                        raise IndexError("row %d outside the bank (%d rows)" % (int(term), bank.shape[0]))
+                    rows[q, t] = int(term)
+                else:
+                    v = np.asarray(term.detach().cpu() if hasattr(term, "detach") else term, dtype=np.float32).reshape(-1)
+                    if v.shape[0] != dim:
+                        raise ValueError("query vector has %d elements, the bank has %d columns" % (v.shape[0], dim))
+                    if vecs is None:
+                        vecs = np.zeros((n, mt, dim), dtype=np.float32)
+                    vecs[q, t] = v
+                    rows[q, t] = -2
+        out = torch.empty((n, dim), dtype=torch.float32, device=self.dev)
+        d_rows, d_w = self.to_device(rows, torch.int32), self.to_device(weights, torch.float32)
+        d_vecs = None if vecs is None else self.to_device(vecs, torch.float32)
+        self._check(self.lib.c2v_compose_queries(self.h, bank.data_ptr(), int(bank.shape[0]), dim, d_rows.data_ptr(),
+                                                 d_w.data_ptr(), _ptr(d_vecs), n, mt, out.data_ptr(), self._stream()))
+        return out
+
+    def nearest(self, bank, queries, k: int, exclude=None):
+        """Cosine top-k of the rows of `bank` (device [rows, dim] float32) for each query (device [n, dim]):
+        (idx int32 [n, k], val float32 [n, k]) device tensors, score descending, ties to the lower row; slots beyond
+        the available results hold -1 / -inf.  exclude: [n, <= 16] row ids never returned (-1 = padding)."""
+        torch = self.torch
+        bank = bank if bank.is_contiguous() else bank.contiguous()
+        queries = self.to_device(queries, torch.float32)
+        if queries.dim() == 1:
+            queries = queries.view(1, -1)
+        n, dim = int(queries.shape[0]), int(bank.shape[1])
+        ex, n_ex = None, 0
+        if exclude is not None:
+            ex = self.to_device(exclude, torch.int32)
+            if ex.dim() != 2 or ex.shape[0] != n:
+                raise ValueError("exclude must be [n, n_exclude]")
+            n_ex = int(ex.shape[1])
+            if n_ex == 0:
+                ex = None
+        idx = torch.empty((n, k), dtype=torch.int32, device=self.dev)
+        val = torch.empty((n, k), dtype=torch.float32, device=self.dev)
+        nbytes = int(self.lib.c2v_nearest_scratch_bytes(int(bank.shape[0]), n, int(k)))
+        scratch = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=self.dev)
+        self._check(self.lib.c2v_nearest(self.h, bank.data_ptr(), int(bank.shape[0]), dim, queries.data_ptr(), n, int(k),
+                                         _ptr(ex), n_ex, idx.data_ptr(), val.data_ptr(), scratch.data_ptr(), nbytes,
+                                         self._stream()))
         return idx, val
 
     def loss(self, code_vec, target):

@@ -166,6 +166,40 @@ int c2v_forward(c2v_engine* e, const int32_t* src, const int32_t* path, const in
 int c2v_topk(c2v_engine* e, const float* code_vec, int32_t B, int32_t* idx, float* val,
              int32_t normalize, void* stream);
 
+/* ---- Nearest-neighbour search: gensim's KeyedVectors.most_similar on a device-resident matrix -----------
+ * What the reference README runs on the --save_t2v / --save_w2v text files (README.md:236-251), and the search
+ * of a code-vector corpus (--export_code_vectors, c2v_predict_batch_host) for the methods closest to a snippet.
+ * bank: device fp32 [rows, dim], row-major, 16-byte aligned, dim % 4 == 0, dim <= 1024, 1 <= rows < 2^31 -- a bound
+ * table (theta.tgt / tok / path; with "lazy_adam" on, call c2v_sync_tables first, otherwise deferred rows are read
+ * stale) or any caller matrix such as code vectors.  Row norms are computed in the same pass as the dot products
+ * (nothing is cached), in fp32 FFMA.  Neither call uses the workspace or changes engine state, so a search
+ * between two train steps leaves the next step bit-identical.  Both are asynchronous on `stream`.
+ *
+ *   c2v_nearest_scratch_bytes : device scratch c2v_nearest needs for (rows, n, k) (per-CTA candidate lists); 0 when
+ *                               the arguments are out of range.
+ *   c2v_compose_queries       : gensim's query vector, unitvec(mean_t(w_t * x_t)), for n queries of up to
+ *                               max_terms (<= 16) terms each.  term_rows / term_weights: device [n, max_terms];
+ *                               term_rows[q, t] >= 0: x_t = bank row / its norm (a zero row adds nothing);
+ *                               -2: x_t = term_vectors[q, t, :] as given (device [n, max_terms, dim], may be NULL
+ *                               when no -2 occurs); -1 (or a row outside the bank): no term.  weights: +1 for a
+ *                               positive term, -1 for a negative one.  queries: device [n, dim] output; a query
+ *                               with no term or a zero mean is all zeros.
+ *   c2v_nearest               : cosine top-k of n query vectors (device [n, dim], any n: chunked internally)
+ *                               against the bank: idx / val device [n, k], score descending, ties to the lower
+ *                               row.  1 <= k <= 64.  exclude: device [n, n_exclude] row ids never returned for
+ *                               that query (-1 = padding), n_exclude <= 16, NULL when 0.  Zero rows and rows whose
+ *                               score is NaN are never returned; a zero query returns nothing; slots beyond the
+ *                               available results hold idx = -1, val = -inf.  Results do not depend on n or on how
+ *                               the queries are batched.  scratch: 16-byte aligned device memory of at least
+ *                               c2v_nearest_scratch_bytes(rows, n, k) bytes. */
+size_t c2v_nearest_scratch_bytes(int64_t rows, int32_t n, int32_t k);
+int c2v_compose_queries(c2v_engine* e, const float* bank, int64_t rows, int32_t dim, const int32_t* term_rows,
+                        const float* term_weights, const float* term_vectors, int32_t n, int32_t max_terms,
+                        float* queries, void* stream);
+int c2v_nearest(c2v_engine* e, const float* bank, int64_t rows, int32_t dim, const float* queries, int32_t n,
+                int32_t k, const int32_t* exclude, int32_t n_exclude, int32_t* idx, float* val, void* scratch,
+                size_t scratch_bytes, void* stream);
+
 /* Mean sparse-softmax cross entropy of code_vec against `target` without gradients
  * (tensorflow_model.py:226-230).  loss_out: device float[1]. */
 int c2v_loss(c2v_engine* e, const float* code_vec, const int32_t* target, int32_t B,
